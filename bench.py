@@ -5,6 +5,7 @@ KITTI-shaped batches; SURVEY.md 8d defines the inputs and the byte accounting).
     python bench.py --gpus 1 --steps 5 --warmup 3                     # our arm (CUDA)
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
     python bench.py --impl reference ...                              # CPU arm (oracle port of the Ceres path)
+    python bench.py ... --dump-outputs DIR                            # + the last timed step's results as DIR/*.npy
 
 A "step" is one pass of the hot path over one batch: S_local clouds x 20480 points -> on-device
 initial guess + front filter + 60 perturbed inits -> batched LM solves -> arg-min pose per cloud
@@ -47,7 +48,13 @@ def parse_args():
     ap.add_argument("--config2-samples", type=int, default=4096)
     ap.add_argument("--ops", action="store_true", help="also time index_max / ball_query (config 3)")
     ap.add_argument("--ops-only", action="store_true", help="only time index_max / ball_query and print that JSON")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step's register_batch returned (rank 0) as DIR/<name>.npy, so that "
+                         "two builds can be compared output for output on the same seeded inputs")
+    args = ap.parse_args()
+    if args.dump_outputs and (args.impl == "reference" or args.ops_only):
+        ap.error("--dump-outputs dumps the CUDA registration path: it takes neither --impl reference nor --ops-only")
+    return args
 
 
 def workload_shape(args):
@@ -353,6 +360,25 @@ def run_registration_config(torch, frustum, lib, dev, xyz_d, pred_d, n_points, K
             "achieved_GBps": achieved, "frac": achieved / peak, "steps": steps, "warmup": max(warmup, 1), "clocks": clocks}
 
 
+DUMP_MAX_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, arrays):
+    """Write every array as out_dir/<name>.npy, integers as float64 (exact), floats as they are.  If they come to more
+    than DUMP_MAX_BYTES in all, a fixed seeded sample of the leading (per-cloud) axis is written instead, and the
+    sampled row numbers go to sample_rows.npy."""
+    arrays = {k: v if v.dtype in (np.float32, np.float64) else v.astype(np.float64) for k, v in arrays.items()}
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_MAX_BYTES:
+        n = next(iter(arrays.values())).shape[0]
+        rows = np.sort(np.random.default_rng(0).choice(n, max(1, n * (DUMP_MAX_BYTES // 2) // total), replace=False))
+        arrays = {k: v[rows] for k, v in arrays.items()}
+        arrays["sample_rows"] = rows.astype(np.float64)
+    os.makedirs(out_dir, exist_ok=True)
+    for k, v in arrays.items():
+        np.save(os.path.join(out_dir, k + ".npy"), v)
+
+
 _JSON_OUT = None
 
 
@@ -500,6 +526,9 @@ def main():
     ms_total = timed_overlapped(args.steps)
     sampler2.mark_end()
     clocks_overlapped = sampler2.stop() if rank == 0 else None
+    # what the headline's last step returned, copied now: the passes below write into the same result buffers
+    dumped = ({k: v.cpu().numpy() for k, v in outs[(args.steps - 1) % n_bufs].items()}
+              if args.dump_outputs and rank == 0 else None)
     ms_per_step = ms_total / args.steps
     value = n_total / (ms_per_step * 1e-3)
     k_ms = sum(kern_ms) / args.steps
@@ -685,6 +714,8 @@ def main():
     if args.ops and "configs" not in line:
         line["ops"] = bench_ops(torch, dev, peak)
     emit(line)
+    if dumped is not None:
+        dump_outputs(args.dump_outputs, dumped)
     if world > 1:
         dist.barrier()
         dist.destroy_process_group()

@@ -11,6 +11,7 @@ header of frustum_oracle.cpp for what is restated and from where.
 import ctypes
 import math
 import os
+import threading
 from concurrent.futures import ThreadPoolExecutor
 
 import numpy as np
@@ -19,16 +20,18 @@ from . import build as _build
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
 _libs = {}
+_libs_lock = threading.Lock()        # the first callers may be worker threads: one of them builds
 
 STAT_FIELDS = ("iterations", "successful_steps", "unique_evals", "cost_evals", "jac_evals",
                "line_search_steps", "termination", "reserved")
 
 
 def _lib(name):
-    if name not in _libs:
-        out = _build.build()
-        _libs[name] = ctypes.CDLL(os.path.join(out, name))
-    return _libs[name]
+    with _libs_lock:
+        if name not in _libs:
+            out = _build.build()
+            _libs[name] = ctypes.CDLL(os.path.join(out, name))
+        return _libs[name]
 
 
 def _p(a, t):

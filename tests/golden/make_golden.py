@@ -5,7 +5,8 @@ oracle/build_ref.py.  Run in the build container only (the GPU box has no /root/
     python oracle/build_ref.py && python tests/golden/make_golden.py
 
 ball_query has no CPU implementation in the reference, and the solver needs Ceres, so neither has
-a fixture; see tests/test_ops_gpu.py::test_against_reference_kernels for the on-box check.
+a fixture here; tests/golden/make_reference_kernels_golden.py stores the outputs of the reference's
+CUDA kernels instead.
 """
 import os
 import sys

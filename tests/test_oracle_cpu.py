@@ -22,6 +22,18 @@ def test_index_max_oracle_matches_reference_golden():
         np.testing.assert_array_equal(oracle.index_max(z["data"], z["index"], int(z["K"])), z["out"])
 
 
+def test_ops_oracles_match_reference_kernel_outputs():
+    """tests/golden/reference_kernels.npz holds what the reference's own CUDA kernels returned on two seeded inputs
+    (the only reference implementation of ball_query)."""
+    g = np.load(os.path.join(GOLDEN, "reference_kernels.npz"))
+    B, C, N, K = (int(v) for v in g["im_shape"])
+    data, index = syn.make_index_max_inputs(int(g["im_seed"]), B, C, N, K)
+    np.testing.assert_array_equal(oracle.index_max(data, index, K), g["im_out"])
+    B, M, N, K = (int(v) for v in g["bq_shape"])
+    dist, radius = syn.make_ball_query_inputs(int(g["bq_seed"]), B, M, N, K)
+    np.testing.assert_array_equal(oracle.ball_query(dist, radius, K), g["bq_out"])
+
+
 def test_index_max_oracle_vs_independent_restatement():
     data, index = syn.make_index_max_inputs(3, 2, 4, 500, 8)
     got = oracle.index_max(data, index, 8)
